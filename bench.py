@@ -77,7 +77,9 @@ def _api(operators):
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=400)
+    ap.add_argument("--steps", type=int, default=400,
+                    help="timed steps of the headline and of the end-to-end loop; the side figures beside them (other "
+                         "operator set, reference comparators) time their own fixed counts and report them")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference", "refgpu"])
     ap.add_argument("--config", default="c2")
@@ -112,7 +114,15 @@ def parse():
     ap.add_argument("--no-graphs", action="store_true", help="pipelined trainer without CUDA-graph capture (debug / A-B)")
     ap.add_argument("--fused", action="store_true",
                     help="render through gsplat.fused.render_gaussians (caller-modified 'next' path) instead of the drop-in operators")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one left the caller (rank 0): the loss and every trained "
+                         "parameter as DIR/<name>.npy (float32, at most 64 MB in all: a fixed, seeded sample of the "
+                         "Gaussians beyond that; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
     if args.sh_chunks is None:
         args.sh_chunks = 1
     return args
@@ -246,6 +256,37 @@ def run_cpu_arm(args, one_shot=False):
 
 
 # ------------------------------------------------------------------------------------------------ GPU arms
+
+DUMP_LIMIT = 64_000_000 - (64 << 10)  # 64 MB, less room for the .npy headers
+
+
+def dump_outputs(out_dir, model, loss):
+    """What a caller of the timed path holds after its last step, as float32 `out_dir/<name>.npy`: `loss` and every
+    trained parameter of the FlatGaussians model (its per-Gaussian views by name, `cam_vel` = the optimised camera
+    velocities).  The inputs are seeded, so two builds run with the same arguments can be compared file by file.  When
+    the whole set would pass 64 MB (from about 270k Gaussians on), every per-Gaussian parameter is written for the same
+    rows only: numpy's default_rng(0).choice(N, rows, replace=False), sorted, with as many rows as fit -- the same rows in
+    every run of the same workload.  `loss` and `cam_vel` are always whole."""
+    import numpy as np
+    import torch
+
+    whole = {"loss": loss.reshape(())}
+    if model.cam_vel is not None:
+        whole["cam_vel"] = model.cam_vel
+    per_gaussian = {k: v.detach().float() for k, v in model.params.items()}
+    n = model.N
+    whole_bytes = sum(4 * v.numel() for v in whole.values())
+    row_bytes = sum(4 * v[0].numel() for v in per_gaussian.values())
+    rows = (DUMP_LIMIT - whole_bytes) // row_bytes
+    if rows < n:
+        idx = np.sort(np.random.default_rng(0).choice(n, size=rows, replace=False))
+        idx = torch.from_numpy(idx).to(model.flat.device)
+        per_gaussian = {k: v[idx] for k, v in per_gaussian.items()}
+    arrays = dict(per_gaussian, **{k: v.detach().float() for k, v in whole.items()})
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v.cpu().numpy())
+
 
 class ClockSampler:
     """nvidia-smi clocks + throttle reasons sampled every 200 ms during the timed region."""
@@ -528,11 +569,13 @@ def run_gpu_arm(args):
     l0 = lib.b200_launch_count() + (trainer.graph_kernel_launches if pipelined else 0)
     evs[0].record()
     for k in range(args.steps):
-        stepper.step(n_warm + k)
+        loss = stepper.step(n_warm + k)
         if pipelined and k == args.steps - 1:
             trainer.finish()  # the last step's SH update (side stream) belongs to the timed region
         evs[k + 1].record()
     barrier()
+    if args.dump_outputs and rank == 0:  # now: the measurements below train the same model further
+        dump_outputs(args.dump_outputs, model, loss)
     launches = (lib.b200_launch_count() + (trainer.graph_kernel_launches if pipelined else 0) - l0) / args.steps
     ms = evs[0].elapsed_time(evs[-1]) / args.steps
     per_step = sorted(evs[k].elapsed_time(evs[k + 1]) for k in range(args.steps))
@@ -627,7 +670,7 @@ def run_gpu_arm(args):
 
     # ---- end to end: host buffers in, loss out, every step (pinned uint8 image + camera H2D, loss D2H)
     cam_host = [torch.cat([c["viewmat"].reshape(-1), c["lin_vel"], c["ang_vel"], c["cam_pos"]]).pin_memory() for c in my]
-    e2e_steps = max(20, args.steps)  # (wall-clock timed: enough steps that filling the prefetch pipeline is noise)
+    e2e_steps = args.steps  # (wall-clock timed: at a few steps, filling the prefetch pipeline shows in the figure)
 
     # double-buffered prefetch on a copy stream (gsplat.data.ImagePrefetcher: what a datamanager does -- pinned uint8
     # image + camera floats), the loss of step k-1 is read back while step k is already queued; every step's inputs cross

@@ -55,3 +55,47 @@ def test_cpu_baseline_imports_survive_the_reference_gpu_helpers():
             "assert hasattr(sys.modules['oracle'], '__path__'); print('ok', O.__name__)")
     r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, capture_output=True, text=True, timeout=300)
     assert r.returncode == 0 and "ok oracle.oracle" in r.stdout, r.stderr[-800:]
+
+
+def _stand_in_model(n, layout):
+    """The parameter shapes of gsplat.dp.FlatGaussians (SH degree 3, 16 camera rows) over one flat buffer; every row of
+    every per-Gaussian parameter starts with its Gaussian's index."""
+    import types
+
+    import torch
+
+    widths = dict(means=3, log_scales=3, quats=4, opacity_logit=1)
+    widths.update(sh=48) if layout == "block" else widths.update(sh_dc=3, sh_rest=45)
+    flat = torch.zeros(n * sum(widths.values()))
+    params, off = {}, 0
+    for name, w in widths.items():
+        params[name] = flat[off:off + n * w].view(n, w)
+        params[name][:, 0] = torch.arange(n, dtype=torch.float32)
+        off += n * w
+    return types.SimpleNamespace(N=n, flat=flat, params=params, cam_vel=torch.ones(16, 6))
+
+
+def test_dump_outputs_stays_under_64_mb_with_the_same_rows(tmp_path):
+    """bench.py --dump-outputs at the largest configs (c5: 2M Gaussians): every per-Gaussian parameter is written for one
+    seeded set of rows, the loss and the camera velocities whole, under 64 MB, identically in two calls."""
+    import numpy as np
+    import torch
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    for layout in ("split", "block"):
+        model = _stand_in_model(2_000_000, layout)
+        dirs = [tmp_path / f"{layout}{k}" for k in range(2)]
+        for d in dirs:
+            bench.dump_outputs(str(d), model, torch.tensor(0.25))
+        names = sorted(os.listdir(dirs[0]))
+        assert names == sorted([k + ".npy" for k in model.params] + ["loss.npy", "cam_vel.npy"])
+        assert sum(os.path.getsize(dirs[0] / f) for f in names) <= 64_000_000
+        out = {f[:-4]: np.load(dirs[0] / f) for f in names}
+        assert all(np.array_equal(out[f[:-4]], np.load(dirs[1] / f)) for f in names)
+        assert out["loss"] == np.float32(0.25) and np.array_equal(out["cam_vel"], np.ones((16, 6), np.float32))
+        rows = out["means"][:, 0]
+        assert 0 < rows.size < 2_000_000 and np.all(np.diff(rows) > 0)
+        for k in model.params:
+            assert out[k].dtype == np.float32 and np.array_equal(out[k][:, 0], rows), k

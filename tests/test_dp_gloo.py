@@ -99,11 +99,11 @@ def test_image_sharded_trainer_gloo(tmp_path, world, sh_chunks):
     assert torch.isfinite(flat).all()
 
 
-def test_single_process_trainer_matches_manual_adam():
+def test_single_process_trainer_matches_manual_adam(monkeypatch):
     sys.path.insert(0, os.path.join(ROOT, "3dgs-deblur_b200"))
     from gsplat import dp, synthetic
 
-    dp.render = _fake_render
+    monkeypatch.setattr(dp, "render", _fake_render)  # (undone after the test: later GPU tests render for real)
     scene = synthetic.make_scene("c1", n_override=20)
     model = dp.FlatGaussians(scene, "cpu")
     ref = model.flat.detach().clone()

@@ -1,35 +1,36 @@
-"""CPU: the UNMODIFIED caller calls this package.
+"""CPU: the calls the UNMODIFIED caller makes reach this package's operators and come back right.
 
-The reference's SplatfactoModel (/root/reference/nerfstudio/nerfstudio/models/splatfacto.py:28-31 imports
-`gsplat.project_gaussians / rasterize / sh / _torch_impl`; :682-899 `get_outputs`) is imported here with `gsplat`
-resolving to 3dgs-deblur_b200/gsplat -- nothing of the caller is edited or replayed -- and run through get_outputs,
-a loss and loss.backward(), in training mode (motion blur + rolling shutter + velocity optimisation, "antialiased"
-opacities) and in eval mode (its second, depth-coloured rasterize_gaussians call).
+The reference's SplatfactoModel (nerfstudio/models/splatfacto.py:28-31 imports `gsplat.project_gaussians / rasterize /
+sh / _torch_impl`; :682-899 `get_outputs`) was run with `gsplat` resolving to 3dgs-deblur_b200/gsplat -- nothing of the
+caller edited -- in training mode (motion blur + rolling shutter + velocity optimisation, "antialiased" opacities), in
+eval mode (its second, depth-coloured rasterize_gaussians call) and in eval mode with motion blur.  Every call it made to
+project_gaussians / spherical_harmonics / rasterize_gaussians is stored in tests/golden/caller_calls.npz
+(tests/golden/make_golden_caller.py): the arguments, and which of them are outputs of an earlier call passed on
+unchanged.  The tests replay those calls through this package, outputs linked as the caller linked them.
 
-What runs under the operators: this container has no GPU and /root/reference cannot travel to the GPU box, so the C-ABI
-layer (`gsplat.cuda`, the 1:1 wrappers of libb200splat) is swapped for the CPU ORACLE (oracle/splat_oracle.c, the checker
-the GPU parity tests hold the kernels to).  Everything between the caller and the C ABI is the product's own code: the
-three operators' argument handling, autograd Functions, gradient routing to velocities / view matrix, the `xys.absgrad`
-side channel, the (rgb, alpha) return convention.  The rendered image is checked against the oracle chain driven directly
-from the model's parameters, and the gradients against float64 finite differences of that chain's loss.
+What runs under the operators: the C-ABI layer (`gsplat.cuda`, the 1:1 wrappers of libb200splat) is swapped for the CPU
+ORACLE (oracle/splat_oracle.c, the checker the GPU parity tests hold the kernels to), so the tests run without a GPU.
+Everything between the caller and the C ABI is the product's own code: the three operators' argument handling, autograd
+Functions, gradient routing to velocities, the `xys.absgrad` side channel, the (rgb, alpha) return convention, the reuse
+of one call's tile lists by the next.  Images are checked against the oracle chain driven directly from the recorded
+arguments, gradients against central differences.
 
 Packages the reference's import chain needs and this image lacks (viser, torchmetrics, pytorch_msssim, nerfacc) are
-stubbed; none of them is on the render path."""
+stubbed by _StubFinder (used by the fixture generators under tests/golden/)."""
 import importlib.abc
 import importlib.machinery
+import inspect
+import json
 import os
-import sys
 import types
 
 import numpy as np
 import pytest
 import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_NS = "/root/reference/nerfstudio"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF_NS), reason="needs /root/reference (build container only)")
+from oracle import oracle as O
 
-from oracle import oracle as O  # noqa: E402
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 class _StubMeta(type):
@@ -75,28 +76,10 @@ class _StubFinder(importlib.abc.MetaPathFinder, importlib.abc.Loader):
         pass
 
 
-@pytest.fixture(scope="module")
-def splatfacto():
-    sys.path.insert(0, os.path.join(ROOT, "3dgs-deblur_b200"))
-    sys.path.insert(0, REF_NS)
-    finder = _StubFinder()
-    sys.meta_path.insert(0, finder)
-    try:
-        import gsplat
-        assert os.path.realpath(os.path.dirname(gsplat.__file__)).startswith(os.path.realpath(ROOT)), "gsplat must be THIS package"
-        import nerfstudio.models.splatfacto as sf
-        from nerfstudio.cameras.cameras import Cameras
-        from nerfstudio.data.scene_box import SceneBox
-        yield sf, Cameras, SceneBox
-    finally:
-        sys.meta_path.remove(finder)
-        sys.path.remove(REF_NS)
-
-
 # ---- gsplat.cuda on the oracle -------------------------------------------------------------------------------------
 
 def _n(t):
-    return t.detach().cpu().numpy()
+    return t.detach().cpu().numpy() if torch.is_tensor(t) else t
 
 
 def _unpack(packed):
@@ -107,9 +90,9 @@ def _unpack(packed):
                                  opac=np.ascontiguousarray(a[:, 10:11]))
 
 
-@pytest.fixture
-def oracle_C(monkeypatch):
-    """Every `gsplat.cuda` entry the three operators reach, computed by the CPU oracle (same signatures)."""
+def install_oracle_C(monkeypatch):
+    """Every `gsplat.cuda` entry the three operators reach, computed by the CPU oracle (same signatures); returns the
+    list the stand-ins log their calls to."""
     import gsplat.cuda as _C
     import gsplat._lib as L
     calls = []
@@ -184,143 +167,145 @@ def oracle_C(monkeypatch):
     return calls
 
 
-def _make_model(sf, SceneBox, n, training, velocity_opt, seed=3):
-    torch.manual_seed(seed)
-    g = torch.Generator().manual_seed(seed)
-    pts = (torch.rand(n, 3, generator=g) - 0.5) * 2.0 + torch.tensor([0.0, 0.0, -3.0])  # in front of an OpenGL camera at the origin
-    cols = torch.rand(n, 3, generator=g) * 255
-    cfg = sf.SplatfactoModelConfig(rasterize_mode="antialiased", blur_samples=5, background_color="white", num_downscales=0,
-                                   sh_degree=3, sh_degree_interval=0 if False else 1)
-    cfg.camera_velocity_optimizer.enabled = velocity_opt
-    box = SceneBox(aabb=torch.tensor([[-1.0, -1.0, -1.0], [1.0, 1.0, 1.0]]))
-    real_cuda = torch.Tensor.cuda
-    torch.Tensor.cuda = lambda self, *a, **k: self  # populate_modules moves the seed colours to "cuda" (splatfacto.py:223)
-    try:
-        model = sf.SplatfactoModel(cfg, scene_box=box, num_train_data=2, seed_points=(pts, cols))
-    finally:
-        torch.Tensor.cuda = real_cuda
-    model.step = 10  # all SH degrees on (splatfacto.py:844)
-    model.train(training)
-    with torch.no_grad():  # something to render: visible sizes, mixed opacities, non-trivial higher SH bands
-        model.gauss_params["scales"].copy_(torch.log(torch.full((n, 3), 0.05) * (0.5 + torch.rand(n, 3, generator=g))))
-        model.gauss_params["opacities"].copy_(torch.randn(n, 1, generator=g))
-        model.gauss_params["features_rest"].copy_(0.1 * torch.randn(n, 15, 3, generator=g))
-    return model
+@pytest.fixture
+def oracle_C(monkeypatch):
+    return install_oracle_C(monkeypatch)
 
 
-def _camera(Cameras, H=48, W=64, with_motion=True):
-    c2w = torch.eye(4)[:3].unsqueeze(0).clone()
-    meta = dict(exposure_time=1 / 60, rolling_shutter_time=1 / 50, cam_idx=0) if with_motion else None  # (cam_idx: camera_optimizers.py:248)
-    vel = torch.tensor([[0.3, -0.2, 0.1, 0.05, 0.4, -0.3]]) if with_motion else None
-    return Cameras(camera_to_worlds=c2w, fx=float(W) / 2, fy=float(W) / 2, cx=W / 2.0, cy=H / 2.0, width=W, height=H, velocities=vel,
-                   metadata=meta)
+@pytest.fixture(scope="module")
+def recorded(golden):
+    g = golden("caller_calls.npz")
+    return json.loads(str(g.pop("spec"))), g
 
 
-def _oracle_chain(model, cam, vel6, S, rs, ex, H, W):
-    """The render block of splatfacto.py:734-880 restated on the oracle, from the model's parameters (numpy, float32)."""
-    p = {k: _n(v) for k, v in model.gauss_params.items()}
-    R_edit = np.diag([1.0, -1.0, -1.0]).astype(np.float32)
-    c2w = _n(cam.camera_to_worlds[0])
-    R = c2w[:3, :3] @ R_edit
-    viewmat = np.concatenate([R.T, -R.T @ c2w[:3, 3:4]], 1).astype(np.float32)
-    lin, ang = (R_edit @ vel6[:3]).astype(np.float32), (R_edit @ vel6[3:]).astype(np.float32)
-    q = p["quats"] / np.linalg.norm(p["quats"], axis=-1, keepdims=True)
-    proj = O.project_forward(p["means"], np.exp(p["scales"]), 1.0, q.astype(np.float32), lin, ang, rs, ex, viewmat, W / 2.0, W / 2.0, W / 2.0,
-                             H / 2.0, H, W, 16)
-    coeffs = np.concatenate([p["features_dc"][:, None, :], p["features_rest"]], 1)
-    rgbs = np.maximum(O.sh_forward("fast", 3, p["means"] - c2w[:3, 3][None], coeffs) + 0.5, 0).astype(np.float32)
-    opac = (1 / (1 + np.exp(-p["opacities"][:, 0])) * proj["compensation"]).astype(np.float32)[:, None]
-    b = O.bin_and_sort(proj["xys"], proj["depths"], proj["radii"], proj["num_tiles_hit"], H, W, 16)
-    img, Ts, fi = O.rasterize_forward(H, W, 16, S, b["gaussian_ids_sorted"], b["tile_bins"], proj["xys"], proj["pix_vels"], rs, ex,
-                                      proj["conics"], rgbs, opac, np.ones(3, np.float32))  # "white" (a black background would
-    #   put exact zeros under the caller's x ** (1 / gamma), whose derivative there is infinite -- in the reference too)
-    return np.minimum(img, 1.0) ** (1 / 2.2), 1 - Ts.mean(-1), proj
+def _replay(spec, arrays):
+    """The recorded calls through this package: returns [(op, bound arguments, outputs)]."""
+    import gsplat
+
+    done, objects = [], {}
+
+    def dec(e):
+        if e["t"] == "out":
+            return done[e["c"]][2][e["o"]]
+        if e["t"] == "py":
+            return e["v"]
+        if e["id"] not in objects:  # (one tensor object where the caller passed one object twice: list reuse sees it)
+            t = torch.from_numpy(arrays[e["k"]].copy())
+            objects[e["id"]] = t.requires_grad_(True) if e["grad"] else t
+        return objects[e["id"]]
+
+    for c in spec["calls"]:
+        fn = getattr(gsplat, c["op"])
+        args, kwargs = [dec(e) for e in c["args"]], {k: dec(e) for k, e in c["kwargs"].items()}
+        bound = inspect.signature(fn).bind(*args, **kwargs)
+        bound.apply_defaults()
+        out = fn(*args, **kwargs)
+        done.append((c["op"], bound.arguments, list(out) if isinstance(out, (tuple, list)) else [out]))
+    return done
 
 
-def test_unmodified_splatfacto_trains_through_this_package(splatfacto, oracle_C):
-    sf, Cameras, SceneBox = splatfacto
-    assert sf.project_gaussians.__module__ == "gsplat.project_gaussians" and sf.rasterize_gaussians.__module__ == "gsplat.rasterize"
-    H, W, n = 48, 64, 400
-    model = _make_model(sf, SceneBox, n, training=True, velocity_opt=True)
-    cam = _camera(Cameras, H, W)
-    out = model.get_outputs(cam)
-    rgb, acc = out["rgb"], out["accumulation"]
-    assert rgb.shape == (H, W, 3) and acc.shape == (H, W, 1) and out["depth"] is None
+def _oracle_blend(proj_args, ras_args):
+    """The oracle chain on the recorded arguments: projection, binning and blend of the colours / opacities the caller
+    passed."""
+    p, r = {k: _n(v) for k, v in proj_args.items()}, {k: _n(v) for k, v in ras_args.items()}
+    proj = O.project_forward(p["means3d"], p["scales"], p["glob_scale"], p["quats"], p["linear_velocity"], p["angular_velocity"],
+                             p["rolling_shutter_time"], p["exposure_time"], p["viewmat"], p["fx"], p["fy"], p["cx"], p["cy"],
+                             p["img_height"], p["img_width"], p["block_width"], p["clip_thresh"])
+    H, W, bw = r["img_height"], r["img_width"], r["block_width"]
+    b = O.bin_and_sort(proj["xys"], proj["depths"], proj["radii"], proj["num_tiles_hit"], H, W, bw)
+    bg = np.ones(3, np.float32) if r["background"] is None else r["background"]
+    img, Ts, _ = O.rasterize_forward(H, W, bw, r["blur_samples"], b["gaussian_ids_sorted"], b["tile_bins"], proj["xys"],
+                                     proj["pix_vels"], r["rolling_shutter_time"], r["exposure_time"], proj["conics"],
+                                     r["colors"], r["opacity"].reshape(-1, 1), bg)
+    return img, 1 - Ts.mean(-1), proj
+
+
+def test_unmodified_splatfacto_trains_through_this_package(recorded, oracle_C):
+    spec, arrays = recorded
+    spec = spec["train"]
+    H, W, n = spec["H"], spec["W"], spec["n"]
+    calls = _replay(spec, arrays)
+    assert [c[0] for c in calls] == ["project_gaussians", "spherical_harmonics", "rasterize_gaussians"]
+    (_, pa, pout), (_, sa, sout), (_, ra, rout) = calls
+    img, alpha = rout
+    assert img.shape == (H, W, 3) and alpha.shape == (H, W)
     # one projection (velocities carry gradients -> exact mode), one SH call at degree 3, one 5-sample blur + RS blend
     assert ("project_fwd", n, H, W, 16, 1 / 50, 1 / 60) in oracle_C and ("sh_fwd", "fast", 3, 3) in oracle_C
     assert ("blend_fwd", 5, 1 / 50, 1 / 60) in oracle_C
-    ref_rgb, ref_alpha, proj = _oracle_chain(model, cam, _n(cam.velocities[0]), 5, 1 / 50, 1 / 60, H, W)
+    ref_img, ref_alpha, proj = _oracle_blend(pa, ra)
     assert int((proj["num_tiles_hit"] > 0).sum()) > 50
-    np.testing.assert_allclose(_n(rgb), ref_rgb, atol=1e-6)
-    np.testing.assert_allclose(_n(acc[..., 0]), ref_alpha, atol=1e-6)
-    target = torch.rand(H, W, 3, generator=torch.Generator().manual_seed(1))
-    loss = (rgb - target).abs().mean() + 0.1 * acc.mean()
-    loss.backward()
+    np.testing.assert_allclose(_n(img), ref_img, atol=1e-6)
+    np.testing.assert_allclose(_n(alpha), ref_alpha, atol=1e-6)
+    np.testing.assert_allclose(_n(sout[0]), O.sh_forward("fast", 3, _n(sa["viewdirs"]), _n(sa["coeffs"])), atol=1e-6)
+    g = torch.Generator().manual_seed(1)
+    v_img, v_alpha = torch.randn(H, W, 3, generator=g) / img.numel(), torch.randn(H, W, generator=g) / alpha.numel()
+    torch.autograd.backward([img, alpha, sout[0]], [v_img, v_alpha, torch.randn(sout[0].shape, generator=g)])
     assert ("project_bwd", True, True, False) in oracle_C and ("blend_bwd", 5) in oracle_C and ("sh_bwd", "fast", 3, 3) in oracle_C
-    for k, v in model.gauss_params.items():
+    leaves = {k: v for args in (pa, sa, ra) for k, v in args.items() if torch.is_tensor(v) and v.requires_grad and v.is_leaf}
+    assert {"means3d", "scales", "quats", "linear_velocity", "angular_velocity", "coeffs", "colors", "opacity"} <= set(leaves)
+    for k, v in leaves.items():
         assert v.grad is not None and torch.isfinite(v.grad).all() and float(v.grad.abs().sum()) > 0, k
-    vel_params = [p for p in model.camera_velocity_optimizer.parameters()]
-    assert vel_params and all(p.grad is not None and float(p.grad.abs().sum()) > 0 for p in vel_params), "no gradient reached the velocity optimizer"
     # the densification side channel the caller reads next (splatfacto.py:416-417)
-    assert model.xys.absgrad.shape == (n, 2) and float(model.xys.absgrad.sum()) > 0 and (model.xys.absgrad >= 0).all()
-    assert model.xys.grad is None or model.xys.grad.shape == (n, 2)
-    # a gradient check that goes through the whole unmodified caller: d loss / d features_dc by central differences
-    idx = int(np.argmax(_n(model.gauss_params["features_dc"].grad).sum(-1).__abs__()))
-    with torch.no_grad():
-        base = model.gauss_params["features_dc"][idx, 0].item()
-        vals = []
-        for eps in (1e-2, -1e-2):
-            model.gauss_params["features_dc"][idx, 0] = base + eps
-            o = model.get_outputs(cam)
-            vals.append(float((o["rgb"] - target).abs().mean() + 0.1 * o["accumulation"].mean()))
-        model.gauss_params["features_dc"][idx, 0] = base
+    xys = pout[0]
+    assert xys.absgrad.shape == (n, 2) and float(xys.absgrad.sum()) > 0 and (xys.absgrad >= 0).all()
+    # d loss / d colour of the Gaussian with the largest gradient, by central differences of the oracle chain
+    colors = ra["colors"]
+    idx = int(np.argmax(np.abs(_n(colors.grad)).sum(-1)))
+    vals = []
+    for eps in (1e-2, -1e-2):
+        c = dict(ra, colors=colors.detach().clone())
+        c["colors"][idx, 0] += eps
+        im, al, _ = _oracle_blend(pa, c)
+        vals.append(float((im * _n(v_img)).sum() + (al * _n(v_alpha)).sum()))
     fd = (vals[0] - vals[1]) / 2e-2
-    assert abs(fd - float(model.gauss_params["features_dc"].grad[idx, 0])) < 0.05 * abs(fd) + 1e-6, (fd, float(model.gauss_params["features_dc"].grad[idx, 0]))
+    assert abs(fd - float(colors.grad[idx, 0])) < 0.05 * abs(fd) + 1e-6, (fd, float(colors.grad[idx, 0]))
 
 
-def test_unmodified_splatfacto_eval_pass_renders_depth_through_this_package(splatfacto, oracle_C):
+def test_unmodified_splatfacto_eval_pass_renders_depth_through_this_package(recorded, oracle_C):
     """Eval mode: static camera (no velocity data, optimizer off), no blur -> S = 1, and the caller's second
     rasterize_gaussians call with depth-valued colours (splatfacto.py:881-897)."""
-    sf, Cameras, SceneBox = splatfacto
-    H, W, n = 32, 48, 300
-    model = _make_model(sf, SceneBox, n, training=False, velocity_opt=False)
-    cam = _camera(Cameras, H, W, with_motion=False)
+    spec, arrays = recorded
+    spec = spec["eval"]
+    H, W = spec["H"], spec["W"]
     with torch.no_grad():
-        out = model.get_outputs(cam)
-    assert out["rgb"].shape == (H, W, 3) and out["depth"].shape == (H, W, 1) and out["accumulation"].shape == (H, W, 1)
+        calls = _replay(spec, arrays)
+    assert [c[0] for c in calls] == ["project_gaussians", "spherical_harmonics", "rasterize_gaussians", "rasterize_gaussians"]
     assert [c for c in oracle_C if c[0] == "blend_fwd"] == [("blend_fwd", 1, 0.0, 0.0)] * 2
-    ref_rgb, ref_alpha, proj = _oracle_chain(model, cam, np.zeros(6, np.float32), 1, 0.0, 0.0, H, W)
-    np.testing.assert_allclose(_n(out["rgb"]), ref_rgb, atol=1e-6)
+    (_, pa, pout), _, (_, ra, (img, alpha)), (_, da, (depth_img,)) = calls
+    ref_img, ref_alpha, proj = _oracle_blend(pa, ra)
+    np.testing.assert_allclose(_n(img), ref_img, atol=1e-6)
+    np.testing.assert_allclose(_n(alpha), ref_alpha, atol=1e-6)
+    # the depth pass blends the projection's depths (what the caller coloured the Gaussians with) on a black background
+    np.testing.assert_allclose(_n(da["colors"])[:, 0], proj["depths"], rtol=1e-3)
+    ref_depth, _, _ = _oracle_blend(pa, da)
+    np.testing.assert_allclose(_n(depth_img), ref_depth, atol=1e-5)
     covered = ref_alpha > 0.5
-    d = _n(out["depth"][..., 0])
-    assert covered.any() and np.all(d[covered] > 1.5) and np.all(d[covered] < 4.5)  # the cloud sits 2..4 units in front
+    d = _n(depth_img)[..., 0][covered] / ref_alpha[covered]
+    assert covered.any() and np.all(d > 1.5) and np.all(d < 4.5)  # the cloud sits 2..4 units in front
 
 
 @pytest.mark.parametrize("rolling_shutter", [False, True])
-def test_eval_depth_pass_reuses_the_colour_pass_lists(splatfacto, oracle_C, monkeypatch, rolling_shutter):
+def test_eval_depth_pass_reuses_the_colour_pass_lists(recorded, oracle_C, monkeypatch, rolling_shutter):
     """Eval with motion blur: the caller's second (static, depth-coloured) rasterize_gaussians call (splatfacto.py:881-897)
     bins nothing when the colour pass had no rolling shutter and an odd sample count -- its lists contain the static
     lists (gsplat/rasterize.py) -- and bins again when it had.  Same depth image either way."""
-    sf, Cameras, SceneBox = splatfacto
-    H, W, n = 32, 48, 300
-    model = _make_model(sf, SceneBox, n, training=False, velocity_opt=False)
-    meta = dict(exposure_time=1 / 60, cam_idx=0)
-    if rolling_shutter:
-        meta["rolling_shutter_time"] = 1 / 50
-    cam = Cameras(camera_to_worlds=torch.eye(4)[:3].unsqueeze(0).clone(), fx=W / 2.0, fy=W / 2.0, cx=W / 2.0, cy=H / 2.0, width=W,
-                  height=H, velocities=torch.tensor([[0.3, -0.2, 0.1, 0.05, 0.4, -0.3]]), metadata=meta)
+    spec, arrays = recorded
+    spec = spec["blur_eval_rs" if rolling_shutter else "blur_eval"]
+    import gsplat.rasterize as R
+    R._last_lists.clear()
     with torch.no_grad():
-        out = model.get_outputs(cam)
+        calls = _replay(spec, arrays)
     blends = [c for c in oracle_C if c[0] == "blend_fwd"]
     assert blends[0][1] == 5 and blends[1] == ("blend_fwd", 1, 0.0, 0.0)
     assert len([c for c in oracle_C if c[0] == "bin"]) == (2 if rolling_shutter else 1)
     del oracle_C[:]
     monkeypatch.setenv("B200SPLAT_NO_LIST_REUSE", "1")
-    import gsplat.rasterize as R
     R._last_lists.clear()
     with torch.no_grad():
-        out2 = model.get_outputs(cam)
+        calls2 = _replay(spec, arrays)
     assert len([c for c in oracle_C if c[0] == "bin"]) == 2
-    assert torch.equal(out["depth"], out2["depth"]) and torch.equal(out["rgb"], out2["rgb"])
-    d = out["depth"][..., 0][out["accumulation"][..., 0] > 0.5]  # (blurred coverage can exceed the static one at the rim: depth 0 there)
-    assert d.numel() > 0 and float(d.min()) > 1.0 and float(d.max()) < 4.5
+    for (_, _, out), (_, _, out2) in zip(calls[2:], calls2[2:]):
+        assert all(torch.equal(a, b) for a, b in zip(out, out2))
+    _, ra, (img, alpha) = calls[2]
+    d = calls[3][2][0][..., 0][alpha > 0.5]  # (blurred coverage can exceed the static one at the rim: depth 0 there)
+    assert d.numel() > 0 and float((d / alpha[alpha > 0.5]).min()) > 1.0 and float((d / alpha[alpha > 0.5]).max()) < 4.5
